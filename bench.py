@@ -377,6 +377,24 @@ def _time_device_steps(torch, dist, world, opt, batch, steps, warmup, flush):
     return float(tt.item()) / steps, launches, wall
 
 
+DUMP_MAX_ELEMS = 1 << 22          # per array: the three parameter-sized arrays stay under 48 MB in all
+
+
+def dump_outputs(out_dir, nn, opt, B):
+    """Writes what the last timed step hands its caller, as <name>.npy (float32): per-utterance cost and skip flag
+    (1.0 = skipped), the summed gradient, the updated parameters and velocity, and the step record {n_valid, sum nll,
+    n_skipped, sweep error flag, gnorm^2, regcost}.  A vector longer than DUMP_MAX_ELEMS is stored as the entries at
+    np.random.RandomState(0).choice(n, DUMP_MAX_ELEMS, replace=False), sorted: the same ones in every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"costs": nn._cost[:B], "skips": (nn._skip[:B] != 0).float(), "grads": nn.grads, "params": nn.params,
+              "velocity": opt._vflat, "step_record": nn.record[:6]}
+    for name, t in arrays.items():
+        a = t.cpu().numpy()
+        if a.size > DUMP_MAX_ELEMS:
+            a = a[np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def _phase_profile(torch, dist, world, rank, opt, batch, flush, nprof):
     """Per-phase device times (CUDA events on the launching stream inside libctcb200), an untimed extra pass."""
     import ctypes
@@ -533,6 +551,8 @@ def run_ours(args, c):
         time.sleep(0.15)
     ms_per_step, launches, t_wall = _time_device_steps(torch, dist, world, opt, batch, args.steps, args.warmup, flush)
     value = Bg / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, nn, opt, Bl)
 
     # ---------------------------------------------------------------- end to end through SGD.run
     e2e_steps = args.steps
@@ -764,12 +784,15 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the C3 / strong-scaling / CTC-sweep sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     c = CONFIGS[args.config]
     if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 3          # bounded sample: a CPU step takes ~0.2-5 s
-            args.warmup = min(args.warmup, 1)
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
         run_reference(args, c)
     else:
         run_ours(args, c)

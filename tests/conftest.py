@@ -45,6 +45,12 @@ def golden_rnn():
 
 
 @pytest.fixture(scope="session")
+def golden_ref():
+    import numpy as np
+    return dict(np.load(os.path.join(ROOT, "tests", "golden", "ctc_reference_exact.npz")))
+
+
+@pytest.fixture(scope="session")
 def cuda():
     import torch
     if not torch.cuda.is_available():

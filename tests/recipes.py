@@ -6,6 +6,8 @@ All follow the reference's own eyeball tests (seed 33, legacy np.random streams)
   c1          : BASELINE.json configs[0]                  (T=200, K=62, |l|=30)
   rnnetcpu    : /root/reference/ctc_fast/debug-utils/rnnetcpu.py:181-193 (D=20,T=10,K=6,H=30,N=3,tl=2)
 """
+import hashlib
+
 import numpy as np
 
 
@@ -83,6 +85,68 @@ ALL_CTC = ["time_trials", "ctc_py"] + list(CTC_CASES)
 def golden_stride(K, T):
     """Golden gradients of the big cases are stored for every 8th frame only (fixtures stay small)."""
     return 1 if K * T <= 50000 else 8
+
+
+def grad_digest(grad):
+    """SHA-256 of a float64 gradient in Fortran order, with -0.0 folded into 0.0 and every NaN into one bit
+    pattern: two gradients have the same digest exactly when np.array_equal(a, b, equal_nan=True) holds."""
+    g = np.asfortranarray(grad, dtype=np.float64) + 0.0
+    g[np.isnan(g)] = np.nan
+    return hashlib.sha256(g.tobytes(order="F")).digest()
+
+
+def grad_sample(grad, n=256):
+    """A fixed, seeded sample of n entries of a gradient (all of it when it is smaller), Fortran order."""
+    flat = np.asarray(grad, dtype=np.float64).ravel(order="F")
+    if flat.size <= n:
+        return flat.copy()
+    return flat[np.sort(np.random.RandomState(0).choice(flat.size, n, replace=False))]
+
+
+def random_ctc_cases():
+    """300 random (K, T, |l|) cases incl. T = 1, T = |l|, T < |l|, heavy label repetition and peaked
+    distributions: yields (K, T, |l|, probs float64 K x T Fortran order, seq int32)."""
+    rng = np.random.RandomState(2024)
+    for _ in range(300):
+        K = int(rng.randint(2, 40))
+        T = int(rng.choice([1, 2, 3, 5, 8, 17, 40, 90]))
+        nlab = int(rng.randint(1, max(2, min(T + 3, 25))))
+        scale = float(rng.choice([0.5, 1.0, 4.0, 12.0]))
+        probs = softmax_cols(rng.randn(K, T) * scale).astype(np.float32).astype(np.float64)
+        if rng.rand() < 0.3:
+            seq = np.full(nlab, 1 + rng.randint(K - 1), dtype=np.int32)           # one label repeated
+        else:
+            seq = (1 + rng.randint(0, K - 1, size=nlab)).astype(np.int32)
+        yield K, T, nlab, np.asfortranarray(probs), seq
+
+
+def random_bf_cases():
+    """200 random blank-forced cases: yields (K, T, len(seq), probs float64 K x T Fortran order, seq int32)."""
+    rng = np.random.RandomState(77)
+    for _ in range(200):
+        K = int(rng.randint(2, 30))
+        T = int(rng.choice([1, 2, 4, 9, 33, 70]))
+        L = int(rng.randint(1, 20))
+        probs = softmax_cols(rng.randn(K, T) * float(rng.choice([1.0, 5.0]))).astype(np.float32).astype(np.float64)
+        seq = rng.randint(0, K, size=L).astype(np.int32)
+        if rng.rand() < 0.7:
+            seq[::2] = 0                                                           # the usual interleaved blanks
+        yield K, T, L, np.asfortranarray(probs), seq
+
+
+def best_path_probs():
+    """One-hot K=10 x T=9 probabilities along a path whose labels 1 and 8 the reference drops (ctc_fast.pyx:176-179)."""
+    probs = np.zeros((10, 9))
+    probs[[0, 3, 3, 0, 3, 1, 5, 5, 8], np.arange(9)] = 1.0
+    return np.asfortranarray(probs)
+
+
+def bf_zero_probability_case():
+    """bf_small with an all-zero frame: a zero frame normaliser (ctc_fast_blankforce.pyx:108-110)."""
+    probs, seq = bf_case("bf_small")
+    p64 = np.asfortranarray(probs.astype(np.float64))
+    p64[:, 4] = 0.0
+    return p64, seq
 
 
 def rnnetcpu():

@@ -90,17 +90,28 @@ def test_product_never_imports_the_oracle():
                 assert "oracle" not in txt.replace("# oracle", ""), "%s mentions the oracle" % f
 
 
+_WITHOUT_CUDA = r'''
+import os, sys
+ROOT = %r
+sys.path[:0] = [ROOT, os.path.join(ROOT, "stanford-ctc_b200")]
+import numpy as np, pytest, torch
+assert not torch.cuda.is_available()
+import ctc_fast
+p = np.asfortranarray(np.full((4, 5), 0.25))
+with pytest.raises(RuntimeError):
+    ctc_fast.ctc_loss(p, np.array([1, 2], dtype=np.int32))
+with pytest.raises(ValueError):                       # reference contract checked before the device
+    ctc_fast.ctc_loss(np.ascontiguousarray(p), np.array([1, 2], dtype=np.int32))
+import nnets.brnnet as rnnet
+with pytest.raises(RuntimeError):
+    rnnet.NNet(5, 4, 8, 2, 10, temporalLayer=1)
+'''
+
+
 def test_product_fails_loudly_without_cuda():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("CUDA present")
-    import numpy as np
-    import ctc_fast
-    p = np.asfortranarray(np.full((4, 5), 0.25))
-    with pytest.raises(RuntimeError):
-        ctc_fast.ctc_loss(p, np.array([1, 2], dtype=np.int32))
-    with pytest.raises(ValueError):                       # reference contract checked before the device
-        ctc_fast.ctc_loss(np.ascontiguousarray(p), np.array([1, 2], dtype=np.int32))
-    import nnets.brnnet as rnnet
-    with pytest.raises(RuntimeError):
-        rnnet.NNet(5, 4, 8, 2, 10, temporalLayer=1)
+    """In a process that sees no device (so that a machine with a GPU checks it too)."""
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, "-c", _WITHOUT_CUDA % ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]

@@ -1,5 +1,6 @@
 """CPU tests: the oracle restatements against the reference's golden vectors (tests/golden, produced by
-the unmodified ctc_fast.pyx) and, where oracle/_ref is present, against the reference itself live."""
+the unmodified ctc_fast.pyx), and bit for bit against what the reference itself computed on the same inputs
+(tests/golden/ctc_reference_exact.npz, from tests/golden/gen_ctc_reference_exact.py)."""
 import numpy as np
 import pytest
 
@@ -12,6 +13,12 @@ REL = 1e-12
 def _run(name):
     probs, seq = recipes.ctc_case(name)
     return probs, seq, ctc_oracle.ctc_loss(np.asfortranarray(probs.astype(np.float64)), seq)
+
+
+def _assert_grad_is_reference(grad, golden_ref, key):
+    """Bit-exact: the recorded sample of the reference's gradient value for value, and all of it by digest."""
+    np.testing.assert_array_equal(recipes.grad_sample(grad), golden_ref[key + "/sample"])
+    assert recipes.grad_digest(grad) == golden_ref[key + "/digest"].tobytes(), key
 
 
 @pytest.mark.parametrize("name", recipes.ALL_CTC)
@@ -41,15 +48,15 @@ def test_known_answer_time_trials():
     assert np.abs(grad.sum(axis=0)).max() < 1e-12      # gradient columns sum to zero
 
 
-@pytest.mark.skipif(ctc_oracle.ref_module() is None, reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", recipes.ALL_CTC)
-def test_c_restatement_matches_reference_live(name):
+def test_c_restatement_matches_reference_live(name, golden_ref):
     probs, seq, (nll, grad, skip) = _run(name)
-    r_nll, r_grad, r_skip = ctc_oracle.ref_ctc_loss(np.asfortranarray(probs.astype(np.float64)), seq)
+    key = "ctc/" + name
+    r_nll, r_skip = float(golden_ref[key + "/nll"]), bool(golden_ref[key + "/skip"])
     assert skip == r_skip
     if not skip:
         assert (nll == r_nll) or (np.isinf(nll) and np.isinf(r_nll))
-        assert np.array_equal(grad, r_grad)          # bit-exact: same operation order in float64
+        _assert_grad_is_reference(grad, golden_ref, key)          # bit-exact: same operation order in float64
 
 
 def test_reference_contract_errors():
@@ -58,15 +65,10 @@ def test_reference_contract_errors():
         ctc_oracle.ctc_loss(np.ascontiguousarray(p.astype(np.float64)), s)   # C-ordered: reference raises too
 
 
-def test_best_path_restatement():
-    probs = np.zeros((10, 9))
-    path = [0, 3, 3, 0, 3, 1, 5, 5, 8]         # labels 1 and 8 are dropped by the reference (:176-179)
-    probs[path, np.arange(9)] = 1.0
-    hyp, align = ctc_oracle.decode_best_path(np.asfortranarray(probs))
+def test_best_path_restatement(golden_ref):
+    hyp, align = ctc_oracle.decode_best_path(recipes.best_path_probs())
     assert hyp == [3, 3, 5] and align == [2, 4, 7]
-    if ctc_oracle.ref_module() is not None:
-        rh, ra = ctc_oracle.ref_module().decode_best_path(np.asfortranarray(probs))
-        assert (list(rh), list(ra)) == (hyp, align)
+    assert (golden_ref["best_path/hyp"].tolist(), golden_ref["best_path/align"].tolist()) == (hyp, align)
 
 
 def test_brnn_restatement_matches_golden(golden_brnn):
@@ -169,27 +171,23 @@ def test_blankforce_restatement_matches_golden(name, golden_bf):
     assert abs(np.linalg.norm(grad) - float(golden_bf[name + "/gradnorm"])) <= 1e-10
 
 
-@pytest.mark.skipif(ctc_oracle.ref_module("ctc_fast_blankforce") is None, reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", recipes.ALL_BF)
-def test_blankforce_restatement_matches_reference_live(name):
+def test_blankforce_restatement_matches_reference_live(name, golden_ref):
     probs, seq = recipes.bf_case(name)
     p64 = np.asfortranarray(probs.astype(np.float64))
     nll, grad, skip = ctc_oracle.ctc_loss_blankforce(p64, seq)
-    r_nll, r_grad, r_skip = ctc_oracle.ref_ctc_loss_blankforce(p64, seq)
-    assert skip == r_skip and nll == r_nll and np.array_equal(grad, r_grad)     # bit-exact
+    key = "bf/" + name
+    assert skip == bool(golden_ref[key + "/skip"]) and nll == float(golden_ref[key + "/nll"])
+    _assert_grad_is_reference(grad, golden_ref, key)                                # bit-exact
     hyp = ctc_oracle.decode_best_path_blankforce(p64)
-    assert hyp == list(ctc_oracle.ref_module("ctc_fast_blankforce").decode_best_path(p64))
+    assert hyp == golden_ref[key + "/hyp"].tolist()
 
 
-def test_blankforce_zero_probability_skips():
+def test_blankforce_zero_probability_skips(golden_ref):
     """A zero frame normaliser is the reference's ZeroDivisionError -> skip (ctc_fast_blankforce.pyx:108-110)."""
-    probs, seq = recipes.bf_case("bf_small")
-    p64 = np.asfortranarray(probs.astype(np.float64))
-    p64[:, 4] = 0.0
-    _, _, skip = ctc_oracle.ctc_loss_blankforce(p64, seq)
+    _, _, skip = ctc_oracle.ctc_loss_blankforce(*recipes.bf_zero_probability_case())
     assert skip
-    if ctc_oracle.ref_module("ctc_fast_blankforce") is not None:
-        assert ctc_oracle.ref_ctc_loss_blankforce(p64, seq)[2]
+    assert bool(golden_ref["bf_zero_probability/skip"])
 
 
 @pytest.mark.parametrize("kw", [dict(temporalLayer=2, unidirectional=True), dict(temporalLayer=-1)])
@@ -229,26 +227,15 @@ def test_rnn_variants_match_golden(golden_rnn):
 
 
 # ---- randomised pinning of the restatements against the compiled reference modules ---------------------------
-@pytest.mark.skipif(ctc_oracle.ref_module() is None, reason="oracle/_ref not built")
-def test_c_restatement_equals_reference_on_random_shapes():
-    """300 random (K, T, |l|) cases incl. T = 1, T = |l|, T < |l|, heavy label repetition and peaked
-    distributions: the C restatement must agree with the unmodified ctc_fast.pyx bit for bit (same float64
-    operation order), skip flags included."""
-    rng = np.random.RandomState(2024)
+def test_c_restatement_equals_reference_on_random_shapes(golden_ref):
+    """recipes.random_ctc_cases (T = 1, T = |l|, T < |l|, heavy label repetition, peaked distributions): the C
+    restatement must agree with the unmodified ctc_fast.pyx bit for bit (same float64 operation order), skip flags
+    included."""
+    r_nlls, r_skips, r_digests = golden_ref["random/nll"], golden_ref["random/skip"], golden_ref["random/digest"]
     n_skip = n_inf = 0
-    for case in range(300):
-        K = int(rng.randint(2, 40))
-        T = int(rng.choice([1, 2, 3, 5, 8, 17, 40, 90]))
-        nlab = int(rng.randint(1, max(2, min(T + 3, 25))))
-        scale = float(rng.choice([0.5, 1.0, 4.0, 12.0]))
-        probs = recipes.softmax_cols(rng.randn(K, T) * scale).astype(np.float32).astype(np.float64)
-        if rng.rand() < 0.3:
-            seq = np.full(nlab, 1 + rng.randint(K - 1), dtype=np.int32)           # one label repeated
-        else:
-            seq = (1 + rng.randint(0, K - 1, size=nlab)).astype(np.int32)
-        p = np.asfortranarray(probs)
+    for case, (K, T, nlab, p, seq) in enumerate(recipes.random_ctc_cases()):
         nll, grad, skip = ctc_oracle.ctc_loss(p, seq)
-        r_nll, r_grad, r_skip = ctc_oracle.ref_ctc_loss(p, seq)
+        r_nll, r_skip = float(r_nlls[case]), bool(r_skips[case])
         assert skip == r_skip, (case, K, T, nlab)
         n_skip += skip
         if skip:
@@ -258,25 +245,18 @@ def test_c_restatement_equals_reference_on_random_shapes():
             assert np.isinf(nll)
         else:
             assert nll == r_nll, (case, K, T, nlab, nll, r_nll)
-        assert np.array_equal(grad, r_grad), (case, K, T, nlab)
+        assert recipes.grad_digest(grad) == r_digests[case].tobytes(), (case, K, T, nlab)
+    assert case == len(r_nlls) - 1
     assert n_skip > 0 and n_inf > 0          # the sample did reach the failure and the T < |l| paths
 
 
-@pytest.mark.skipif(ctc_oracle.ref_module("ctc_fast_blankforce") is None, reason="oracle/_ref not built")
-def test_blankforce_restatement_equals_reference_on_random_shapes():
-    rng = np.random.RandomState(77)
-    for case in range(200):
-        K = int(rng.randint(2, 30))
-        T = int(rng.choice([1, 2, 4, 9, 33, 70]))
-        L = int(rng.randint(1, 20))
-        probs = recipes.softmax_cols(rng.randn(K, T) * float(rng.choice([1.0, 5.0]))).astype(np.float32).astype(np.float64)
-        seq = rng.randint(0, K, size=L).astype(np.int32)
-        if rng.rand() < 0.7:
-            seq[::2] = 0                                                           # the usual interleaved blanks
-        p = np.asfortranarray(probs)
+def test_blankforce_restatement_equals_reference_on_random_shapes(golden_ref):
+    r_nlls, r_skips, r_digests = golden_ref["random_bf/nll"], golden_ref["random_bf/skip"], golden_ref["random_bf/digest"]
+    for case, (K, T, L, p, seq) in enumerate(recipes.random_bf_cases()):
         nll, grad, skip = ctc_oracle.ctc_loss_blankforce(p, seq)
-        r_nll, r_grad, r_skip = ctc_oracle.ref_ctc_loss_blankforce(p, seq)
+        r_nll, r_skip = float(r_nlls[case]), bool(r_skips[case])
         assert skip == r_skip, (case, K, T, L)
         if not skip:
             assert (nll == r_nll) or (np.isnan(nll) and np.isnan(r_nll)) or (np.isinf(nll) and np.isinf(r_nll)), (case, nll, r_nll)
-            assert np.array_equal(grad, r_grad, equal_nan=True), (case, K, T, L)
+            assert recipes.grad_digest(grad) == r_digests[case].tobytes(), (case, K, T, L)
+    assert case == len(r_nlls) - 1
